@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 segmentation hot path (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload infer|train] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload infer|train] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Default workload (N=1): BASELINE config[1] -- MobileNetV2UNet bf16 inference, batch 64 per GPU at
@@ -21,6 +21,13 @@ One JSON line on rank 0:
   cpu_baseline  the oracle port of the reference path (fp32, PyTorch CPU) on this box's host cores
 --impl reference: times that CPU path alone: the real reference (/root/reference via the Appendix-D shim) when that
 tree is present, else its restatement oracle/unet_oracle.py (the GPU box has no /root/reference); `kind` says which ran.
+
+--dump-outputs DIR: rank 0 writes what each timed leg returned in its last timed step as DIR/<name>.npy (float32):
+logits (value leg), mask (e2e leg), train_loss and train_params (training leg: the loss and the weights the step updated).
+Inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.  The
+inference arrays repeat bit for bit; the training ones only to rounding (BatchNorm sums depend on atomic order, and Adam's
+normalised update magnifies that in weights whose gradients are near zero: measured on a B200 at 1000 W, two runs of the
+default line differed by up to 5e-4 in train_loss and 4e-3 in train_params).
 """
 import argparse
 import json
@@ -55,7 +62,35 @@ def parse():
     ap.add_argument("--no-train-leg", action="store_true", help="skip the config[2] training leg of the default run")
     ap.add_argument("--no-eager-baseline", action="store_true", help="skip the torch-eager incumbent legs (N=1)")
     ap.add_argument("--sustain-seconds", type=float, default=2.0, help="length of the extra sustained-throughput loop")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of every leg to DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the b200 path; --impl reference has no outputs to dump")
+    return args
+
+
+DUMP_ELEMS = 1 << 22        # float32 values per dumped array (16 MB): the four arrays stay under 64 MB at any batch
+DUMP_SEED = 1234
+
+
+def output_dumper(out_dir, rank):
+    """dump(name, tensor) for --dump-outputs, or None.  A tensor of at most DUMP_ELEMS values is written whole; a larger
+    one as the values at DUMP_ELEMS seeded positions of its flattened form (the same positions for the same shape, in
+    ascending order), so that two runs with the same arguments write comparable arrays."""
+    if not out_dir or rank != 0:
+        return None
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+
+    def dump(name, t):
+        t = t.detach()
+        if t.numel() > DUMP_ELEMS:
+            g = torch.Generator().manual_seed(DUMP_SEED)
+            idx = torch.randint(t.numel(), (DUMP_ELEMS,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    return dump
 
 
 def peaks():
@@ -248,9 +283,10 @@ def main():
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
+    dump = output_dumper(args.dump_outputs, rank)
     if args.workload in ("train", "unet_train"):
         from bench_train import run_train          # training step benchmark lives in its own file
-        return run_train(args, dev, dist, world, rank, peaks(), clocks, emit, shutdown)
+        return run_train(args, dev, dist, world, rank, peaks(), clocks, emit, shutdown, dump)
 
     global H, W
     if args.workload == "infer720":
@@ -303,6 +339,8 @@ def main():
             print("sampler polls (start ms, duration ms): " + " ".join(f"{(a - h0) * 1e3:.1f}/{(b - a) * 1e3:.2f}" for a, b in clocks.poll_log[-12:]),
                   file=sys.stderr)
         clk = clocks.stop() if rank == 0 else None
+        if dump is not None:
+            dump("logits", y)                       # y: the last timed step's result
         # sustained figure: the same loop for >= --sustain-seconds (power/thermals settled), reported beside `value`
         n_sus = max(args.steps, int(args.sustain_seconds * 1e3 / max(ms / args.steps, 1e-3)))
         s0, s1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -373,6 +411,8 @@ def main():
         t1.record()
         barrier()
         ms_e2e = t0.elapsed_time(t1)
+        if dump is not None:
+            dump("mask", mh[(LEAD_IN + args.steps - 1) & 1])      # the host mask of the last timed step
         if E2E_TRACE is not None and rank == 0:
             h0, d0 = E2E_TRACE[0]
             print("e2e trace (step: host issue ms, device done ms): " +
@@ -472,7 +512,7 @@ def main():
         eng._graphs.clear()
         torch.cuda.empty_cache()
         from bench_train import train_leg
-        train = train_leg(args, dev, dist, world, rank)
+        train = train_leg(args, dev, dist, world, rank, dump=dump)
     if rank != 0:
         shutdown(dist)
         return

@@ -17,10 +17,11 @@ TRAIN_BYTES_PER_IMG = 353e6        # SURVEY 8d: MobileNetV2UNet train, bf16 acti
 UNET_BYTES_PER_IMG = 4772e6        # SURVEY 8d: UNet(10) train, bf16 activations, 3x512x1024
 
 
-def train_leg(args, dev, dist, world, rank, unet=False, batch=0, want_breakdown=False, clocks=None):
+def train_leg(args, dev, dist, world, rank, unet=False, batch=0, want_breakdown=False, clocks=None, dump=None):
     """Times the training step three ways (device-resident inputs; end to end from pinned host batches with loss.item()
     every step; for N>1 the same step with the collectives detached = the exposed all-reduce time).  Returns a dict of
-    plain numbers (max over ranks where it matters) + the per-layer trace of one warm eager step."""
+    plain numbers (max over ranks where it matters) + the per-layer trace of one warm eager step.  ``dump`` (bench.py's
+    --dump-outputs) receives the loss and the weights of the last device-resident timed step."""
     import b200seg
     from b200seg import dp, train_path
     H, W = (512, 1024) if unet else (256, 512)
@@ -80,6 +81,9 @@ def train_leg(args, dev, dist, world, rank, unet=False, batch=0, want_breakdown=
     launches_per_step = in_graph + (LAUNCHES[0] - n0) / args.steps      # kernels replayed from the two graphs + launched directly
     clk = clocks.stop() if (clocks is not None and rank == 0) else None
     last_loss = float(loss)
+    if dump is not None:
+        dump("train_loss", loss)
+        dump("train_params", torch.cat([p.detach().reshape(-1) for p in model.parameters()]))
 
     # e2e: host (pinned) fp32 images + int64 labels in, loss.item() out, every step.  Input feed (SURVEY 8f rank 4):
     # non-blocking uploads on a copy stream, one batch ahead -- the upload of batch i+1 overlaps step i although the loss is
@@ -152,9 +156,9 @@ def train_leg(args, dev, dist, world, rank, unet=False, batch=0, want_breakdown=
     return res
 
 
-def run_train(args, dev, dist, world, rank, pk, clocks, emit, shutdown):
+def run_train(args, dev, dist, world, rank, pk, clocks, emit, shutdown, dump=None):
     unet = args.workload == "unet_train"
-    r = train_leg(args, dev, dist, world, rank, unet=unet, batch=args.batch, want_breakdown=True, clocks=clocks)
+    r = train_leg(args, dev, dist, world, rank, unet=unet, batch=args.batch, want_breakdown=True, clocks=clocks, dump=dump)
     rows, tot = r["rows"], r["rows_total"]
     if args.breakdown and rank == 0:
         print(f"{'phase':4s} {'layer':34s} {'ms':>9s} {'share':>6s}", file=sys.stderr)
