@@ -28,6 +28,10 @@ extern "C" {
 typedef struct CUstream_st* b200seg_stream_t;
 
 enum { B200SEG_F32 = 0, B200SEG_BF16 = 1 };
+/* target (label map) dtypes of the validation-metrics entry points */
+enum { B200SEG_I64 = 2, B200SEG_U8 = 3 };
+/* logits layout of b200seg_seg_metrics */
+enum { B200SEG_NCHW = 0, B200SEG_NHWC = 1 };
 enum { B200SEG_ACT_NONE = 0, B200SEG_ACT_RELU = 1, B200SEG_ACT_RELU6 = 2 };
 
 int b200seg_version(void);
@@ -138,6 +142,28 @@ int b200seg_mbconv(const void* x, const void* w_exp, const float* b_exp, const v
  *   x [B,h,w,32] bf16;  w0 bf16 [16][32], b0 f32 [16];  w3 bf16 [16][16] (rows >= C zero), b3 f32 [16];  C <= 16. */
 int b200seg_tail_fused(const void* x, const void* w0, const float* b0, const void* w3, const float* b3, void* out,
                        int out_dtype, uint8_t* mask, int B, int h, int w, int C, b200seg_stream_t s);
+
+/* Validation metrics (the commented-out validation loop of train.py:46-74) accumulated on the device.  Both entry points
+ * ADD into the caller's state (zero it to start):
+ *   confusion int64 [C][C]  row = target class, column = predicted class (argmax, first maximum wins like torch.argmax)
+ *   counts    int64 [2]     [0] += pixels whose target is in [0,C) and not ignore_index; [1] += pixels whose target is
+ *                           neither in range nor ignore_index (nn.CrossEntropyLoss raises on those; the Python layer
+ *                           reports a NaN loss).  A pixel whose target equals ignore_index contributes nothing, also when
+ *                           ignore_index is a class index.
+ *   loss_sum  f64 [1]       += sum over the counted pixels of logsumexp(z) - z[target] (f32 per pixel and per CTA)
+ *   target    [B,2h,2w] (tail) or [B,H,W] of target_dtype B200SEG_I64 (16-byte aligned for the tail) or B200SEG_U8
+ *             (2-byte aligned for the tail); a uint8 label equal to ignore_index is ignored like an int64 one.
+ * b200seg_tail_fused_metrics: the output tail above (same operands, C <= 16) with the metrics taken in its epilogue from the
+ *   same interpolated logits the mask mode compares, so the confusion equals the histogram of that mask exactly; no
+ *   logits tensor is written.
+ * b200seg_seg_metrics: the same metrics over existing logits (f32 | bf16), C <= 64.  layout B200SEG_NCHW: [B,C,H,W]
+ *   (ldc ignored); B200SEG_NHWC: [B,H,W,ldc] with the first C channels valid (UNet's padded logits buffer). */
+int b200seg_tail_fused_metrics(const void* x, const void* w0, const float* b0, const void* w3, const float* b3,
+                               const void* target, int target_dtype, long long ignore_index, int64_t* confusion,
+                               int64_t* counts, double* loss_sum, int B, int h, int w, int C, b200seg_stream_t s);
+int b200seg_seg_metrics(const void* logits, int dtype, int layout, int ldc, const void* target, int target_dtype,
+                        long long ignore_index, int64_t* confusion, int64_t* counts, double* loss_sum, int B, int C, int H,
+                        int W, b200seg_stream_t s);
 
 /* NHWC [B,H,W,ldc] (first C valid) -> NCHW [B,C,H,W] (UNet returns logits at input resolution). */
 int b200seg_nhwc_to_nchw(const void* x, int dtype, int ldc, void* out, int out_dtype, int B, int H, int W,

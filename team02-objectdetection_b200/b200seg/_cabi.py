@@ -14,6 +14,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libb200seg.so")
 
 F32, BF16 = 0, 1
+I64, U8 = 2, 3              # target dtypes of the metrics entry points
+NCHW, NHWC = 0, 1           # logits layouts of b200seg_seg_metrics
 ACT_NONE, ACT_RELU, ACT_RELU6 = 0, 1, 2
 
 _vp, _i, _f, _ll, _d = C.c_void_p, C.c_int, C.c_float, C.c_longlong, C.c_double
@@ -37,6 +39,8 @@ _PROTOS = {
     "b200seg_upsample2x_ac_nchw": [_vp, _i, _i, _vp, _i, _i, _i, _i, _i, _vp],
     "b200seg_upsample2x_ac_argmax": [_vp, _i, _i, _vp, _i, _i, _i, _i, _vp],
     "b200seg_tail_fused": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp],
+    "b200seg_tail_fused_metrics": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _ll, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
+    "b200seg_seg_metrics": [_vp, _i, _i, _i, _vp, _i, _ll, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
     "b200seg_nhwc_to_nchw": [_vp, _i, _i, _vp, _i, _i, _i, _i, _i, _vp],
     "b200seg_maxpool2x2": [_vp, _vp, _i, _i, _i, _i, _i, _vp],
     "b200seg_softmax_ce": [_vp, _vp, _vp, _vp, _f, _vp, _i, _i, _i, _i, _vp],

@@ -360,9 +360,10 @@ class Engine:
             raise RuntimeError(f"input on {x.device} but model on {p0.device}")
 
     # ------------------------------------------------------------------ forward (eval)
-    def _run_step(self, s: Step, env, pk, mode: str, sdt, dense_impl: str, out_dtype, want_mask: bool, out=None):
+    def _run_step(self, s: Step, env, pk, mode: str, sdt, dense_impl: str, out_dtype, want_mask: bool, metrics=None, out=None):
         """Launch the kernel of one fused step; inputs/outputs live in ``env`` by schedule name.  ``out``: existing output
-        buffer (only for the head step, which is launched outside the captured graph into a static buffer)."""
+        buffer (only for the head step, which is launched outside the captured graph into a static buffer).  ``metrics``:
+        (SegmentationMetrics, target): the last step accumulates validation metrics instead of writing an output."""
         if s.op == "stem":
             p = pk[s.name]
             env[s.dst] = ops.conv3x3_smallcin(env[s.src], p["w"], p["b"], s.stride, s.act, sdt, out=out)
@@ -390,6 +391,12 @@ class Engine:
             p = pk[s.parts[2].name + "#mb"]
             env[s.dst] = ops.mbconv(env[s.src], p["w_exp"], p["b_exp"], p["w_dw"], p["b_dw"], p["w_proj"], p["b_proj"],
                                     s.stride, s.res is not None, flags=self.mbconv_flags)
+        elif s.op == "tail" and metrics is not None:
+            p0, p3 = pk[s.parts[0].name], pk[s.parts[1].name]
+            sm, tgt = metrics
+            ops.tail_fused_metrics(env[s.src], p0["w"], p0["b64"], p3["w"], p3["b64"], self.out_ch, tgt, sm.ignore_index,
+                                   sm.confusion, sm.counts, sm.loss_sum)
+            env[s.dst] = None
         elif s.op == "tail":
             p0, p3 = pk[s.parts[0].name], pk[s.parts[1].name]
             env[s.dst] = ops.tail_fused(env[s.src], p0["w"], p0["b64"], p3["w"], p3["b64"], self.out_ch, out_dtype, want_mask, out=out)
@@ -397,6 +404,14 @@ class Engine:
             env[s.dst] = ops.upsample2x_concat(env[s.res], env[s.src])
         elif s.op == "pool":
             env[s.dst] = ops.maxpool2x2(env[s.src])
+        elif s.op in ("final", "to_nchw") and metrics is not None:
+            sm, tgt = metrics
+            if s.op == "final":      # f32 NCHW logits: the values the argmax of predict_mask compares
+                ops.seg_metrics(ops.upsample2x_ac_nchw(env[s.src], self.out_ch, torch.float32), tgt, self.out_ch,
+                                sm.ignore_index, sm.confusion, sm.counts, sm.loss_sum)
+            else:                    # UNet: straight from the NHWC logits buffer, no layout pass
+                ops.seg_metrics(env[s.src], tgt, self.out_ch, sm.ignore_index, sm.confusion, sm.counts, sm.loss_sum, nhwc=True)
+            env[s.dst] = None
         elif s.op == "final":
             if want_mask:
                 env[s.dst] = ops.upsample2x_ac_argmax(env[s.src], self.out_ch, out=out)
@@ -412,9 +427,10 @@ class Engine:
 
     @torch.no_grad()
     def forward_eval(self, x: torch.Tensor, want_mask: bool = False, keep: Optional[dict] = None,
-                     profile: Optional[list] = None, out=None):
+                     profile: Optional[list] = None, out=None, metrics=None):
         """Eval-mode forward.  ``keep`` (dict) receives every intermediate NHWC tensor by schedule name;
         ``profile`` (list) receives (step, start_event, end_event, bytes, flops) per launched kernel.
+        ``metrics`` = (SegmentationMetrics, target): the last step accumulates the validation metrics and returns None.
 
         Steady state (same shape seen ``graph_after`` times, weights unchanged): the first kernel (reads the
         caller's NCHW tensor) and the last one (writes a fresh NCHW result) are launched directly, every
@@ -431,7 +447,7 @@ class Engine:
             raise TypeError(f"input dtype {x.dtype} not supported")
         x = x.contiguous()
         out_dtype = x.dtype
-        args = (pk, mode, sdt, dense_impl, out_dtype, want_mask)
+        args = (pk, mode, sdt, dense_impl, out_dtype, want_mask, metrics)
         steps = self._schedule(mode, dense_impl, x.shape[2], x.shape[3], x.dtype)
 
         if keep is None and profile is None and self.use_graphs and not torch.cuda.is_current_stream_capturing():
@@ -453,7 +469,7 @@ class Engine:
                 self._run_step(ent["tail"], env, *args, out=out)
                 return env["out"]
 
-        env: Dict[str, torch.Tensor] = {"x": x}
+        env: Dict[str, Optional[torch.Tensor]] = {"x": x}
         for s in steps:
             if profile is not None:
                 ev0 = torch.cuda.Event(enable_timing=True); ev0.record()
@@ -469,7 +485,7 @@ class Engine:
     def _capture(self, ent, x, args, steps):
         """Capture steps[1:-1] into a CUDA graph.  Buffers allocated inside the capture come from the
         graph's private pool and stay valid for every replay."""
-        pk, mode, sdt, dense_impl, out_dtype, want_mask = args
+        pk, mode, sdt, dense_impl, out_dtype, want_mask, metrics = args
         head, body, tail = steps[0], steps[1:-1], steps[-1]
         assert head.op in ("stem", "stem_mb1") and tail.op in ("final", "to_nchw", "tail")
         ent["head"] = head
@@ -557,13 +573,15 @@ class Engine:
         return nbytes, flops
 
     # ------------------------------------------------------------------ dispatch
-    def forward(self, x: torch.Tensor, want_mask: bool = False, out=None):
+    def forward(self, x: torch.Tensor, want_mask: bool = False, out=None, metrics=None):
         # every kernel is launched on the current stream of the CURRENT device: make the input's device current for the
         # whole call (model.to("cuda:1") while cuda:0 is current must work like any nn.Module)
         with torch.cuda.device(x.device):
             if self.model.training:
                 if want_mask:
                     raise RuntimeError("predict_mask needs model.eval()")
+                if metrics is not None:
+                    raise RuntimeError("evaluate needs model.eval()")
                 from . import train_path
                 return train_path.forward_train(self, x)
-            return self.forward_eval(x, want_mask, out=out)
+            return self.forward_eval(x, want_mask, out=out, metrics=metrics)

@@ -296,6 +296,57 @@ def tail_fused(x, w0, b0, w3, b3, C: int, out_dtype=None, want_mask: bool = Fals
     return out
 
 
+_TGT = {torch.int64: _cabi.I64, torch.uint8: _cabi.U8}
+
+
+def _metrics_target(target, shape):
+    """int64 | uint8 label map of ``shape``, contiguous and 16-byte aligned for the kernels' vector loads: a non-contiguous
+    or misaligned view (a crop of a larger label map) is copied."""
+    if target.dtype not in _TGT:
+        raise ValueError(f"targets must be int64 or uint8, got {target.dtype}")
+    if tuple(target.shape) != tuple(shape):
+        raise ValueError(f"target shape {tuple(target.shape)} does not match the logits' [B,H,W] {tuple(shape)}")
+    target = target.contiguous()
+    if target.data_ptr() % 16:                   # a view at an odd offset: the 16-byte target loads need an aligned copy
+        target = target.clone()
+    return target
+
+
+def tail_fused_metrics(x, w0, b0, w3, b3, C: int, target, ignore_index: int, confusion, counts, loss_sum):
+    """outconv(32, C) + final_upsample + validation metrics in one kernel (operands as tail_fused): adds the confusion
+    matrix, [valid, invalid] counts and the cross-entropy sum of ``target`` [B,2h,2w] into the int64 / f64 state."""
+    _cuda(x, w0, b0, w3, b3, confusion, counts, loss_sum)
+    B, h, w, cin = x.shape
+    if (x.dtype != torch.bfloat16 or cin != 32 or tuple(w0.shape) != (16, 32) or tuple(w3.shape) != (16, 16)
+            or w0.dtype != torch.bfloat16 or w3.dtype != torch.bfloat16 or b0.numel() < 16 or b3.numel() < 16 or not 1 <= C <= 16):
+        raise ValueError("tail_fused_metrics: expects the MobileNetV2UNet tail (32 -> 16 -> C <= 16 channels, bf16)")
+    target = _metrics_target(target, (B, 2 * h, 2 * w))
+    _cuda(target)
+    check(lib.b200seg_tail_fused_metrics(ptr(x), ptr(w0), ptr(b0), ptr(w3), ptr(b3), ptr(target), _TGT[target.dtype],
+                                         int(ignore_index), ptr(confusion), ptr(counts), ptr(loss_sum), B, h, w, C, _stream()),
+          "tail_fused_metrics")
+
+
+def seg_metrics(logits, target, C: int, ignore_index: int, confusion, counts, loss_sum, nhwc: bool = False):
+    """Validation metrics over existing logits: NCHW [B,C,H,W] (``nhwc`` False) or NHWC [B,H,W,ldc >= C] (f32 | bf16),
+    int64 | uint8 targets [B,H,W]; adds into the int64 / f64 state like tail_fused_metrics."""
+    _cuda(logits, confusion, counts, loss_sum)
+    if logits.dim() != 4:
+        raise ValueError(f"logits must be 4-D, got {tuple(logits.shape)}")
+    if nhwc:
+        B, H, W, ldc = logits.shape
+    else:
+        B, Cl, H, W = logits.shape
+        ldc = 0
+        if Cl != C:
+            raise ValueError(f"logits have {Cl} classes, expected {C}")
+    target = _metrics_target(target, (B, H, W))
+    _cuda(target)
+    check(lib.b200seg_seg_metrics(ptr(logits), _dt(logits), _cabi.NHWC if nhwc else _cabi.NCHW, ldc, ptr(target),
+                                  _TGT[target.dtype], int(ignore_index), ptr(confusion), ptr(counts), ptr(loss_sum),
+                                  B, C, H, W, _stream()), "seg_metrics")
+
+
 def nhwc_to_nchw(x, C: int, out_dtype, out=None):
     _cuda(x)
     B, H, W, ldc = x.shape

@@ -177,6 +177,24 @@ class _EngineModel(nn.Module):
         (a frame loop that hands the mask to another stream keeps two of them instead of allocating per frame)."""
         return self._get_engine().forward(x, want_mask=True, out=out)
 
+    @torch.no_grad()
+    def evaluate(self, x: torch.Tensor, target: torch.Tensor, metrics):
+        """Validation step (the reference's commented-out loop, train.py:46-74): the forward of ``x`` with the loss,
+        argmax and confusion histogram against ``target`` (int64 [B,H,W] CrossEntropyLoss targets, or uint8) accumulated
+        into ``metrics`` (b200seg.SegmentationMetrics) on the device.  No logits tensor is returned (MobileNetV2UNet in
+        bf16 never writes one: the output-tail kernel takes the metrics itself).  Eval mode only; never synchronises
+        with the host.  Returns ``metrics``."""
+        if self.training:
+            raise RuntimeError("evaluate needs model.eval()")
+        if not x.is_cuda:
+            raise RuntimeError("b200seg models run on CUDA (sm_100a) only; got a CPU tensor. "
+                               "There is deliberately no CPU fallback.")
+        if metrics.num_classes != self.output_channels:
+            raise ValueError(f"metrics count {metrics.num_classes} classes, the model outputs {self.output_channels}")
+        metrics._check(x, target)
+        self._get_engine().forward(x, metrics=(metrics, target))
+        return metrics
+
 
 class MobileNetV2UNet(_EngineModel):
     """unet.py:7-51.  NOTE unet.py:12 downloads ImageNet weights; offline that is impossible, so

@@ -3,6 +3,8 @@
 //     outc = outconv(32, C):  1x1 (32->16) + BN + ReLU -> 1x1 (16->C) + bias          (unet.py:108-121, :47)
 //     final_upsample:         bilinear x2, align_corners=True                          (unet.py:30, :49)
 //     [optional]              argmax over the classes -> uint8 mask                    (inference.py:64)
+//     [optional]              validation metrics against targets: confusion histogram, valid / invalid counts and the
+//                             cross-entropy sum (seg_metrics.cuh); no logits leave the chip
 //
 // Unfused these were three launches and two round trips of a 16/10-channel tensor through HBM (64 + 64 + 99 us at
 // batch 64 on the B200: 0.32 / 0.48 / 0.36 of the HBM roofline).  Fused, the kernel reads the 32-channel decoder
@@ -17,7 +19,7 @@
 // straight from global: thread (g, t) of a group loads the 16-byte vector [8t, 8t+8) of pixels g and g+8 -- a fully
 // coalesced 512-byte warp load -- and the K order of the weight fragments is permuted to match), phase 2 interpolates
 // from shared memory with the same association as upsample2x_ac_kernel (vertical blend, then horizontal).
-#include "common.cuh"
+#include "seg_metrics.cuh"
 
 namespace b200 {
 
@@ -37,12 +39,21 @@ __device__ __forceinline__ uint32_t ld_pair(const __nv_bfloat16* p) { return __l
 // x   : NHWC bf16 [B,h,w,32]        w0 : bf16 [16][32] (BN folded)   b0 : f32 [16]
 // w3  : bf16 [16][16] (rows >= C zero)   b3 : f32 [16]
 // out : NCHW [B,C,2h,2w] of TO, or mask uint8 [B,2h,2w]
-template <typename TO, bool ARGMAX>
+// TGT : void, or the target type (int64_t | uint8_t) of the metrics epilogue (tgt [B,2h,2w], state ms; out / mask unused)
+template <typename TGT>
+__device__ __forceinline__ void tail_metrics_phase2(const float* lg, uint32_t* hist, const TGT* __restrict__ tgt, const SegMetricsState& ms,
+                                                    int b, int h, int w, int C, int oy0, int ox0, int yf, int xf, float sch,
+                                                    float scw);
+
+template <typename TO, bool ARGMAX, typename TGT = void>
 __global__ void __launch_bounds__(256)
 tail_fused_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ w0, const float* __restrict__ b0,
                   const __nv_bfloat16* __restrict__ w3, const float* __restrict__ b3, TO* __restrict__ out,
-                  uint8_t* __restrict__ mask, int B, int h, int w, int C, int tiles_x, int tiles_y) {
+                  uint8_t* __restrict__ mask, int B, int h, int w, int C, int tiles_x, int tiles_y,
+                  const void* __restrict__ tgt, SegMetricsState ms) {
+  constexpr bool METRICS = !std::is_void<TGT>::value;
   extern __shared__ float lg[];                   // [C][TAIL_NPX] half-resolution logits of this tile, fp32
+                                                  // (metrics: then the u32 [C][C] histogram and 24 reduction words)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int Ho = 2 * h, Wo = 2 * w;
@@ -79,6 +90,8 @@ tail_fused_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __re
   for (int j = 0; j < 2; ++j)
 #pragma unroll
     for (int e = 0; e < 2; ++e) { bias0[j][e] = __ldg(b0 + j * 8 + 2 * t + e); bias3[j][e] = __ldg(b3 + j * 8 + 2 * t + e); }
+
+  if constexpr (METRICS) seg_hist_zero(reinterpret_cast<uint32_t*>(lg + C * TAIL_NPX), C);   // published by phase 1's barrier
 
   // ---- phase 1: logits of the TAIL_SR x TAIL_SC source pixels ----
   const __nv_bfloat16* xb = x + (long long)b * h * w * 32;
@@ -125,6 +138,12 @@ tail_fused_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __re
       }
   }
   __syncthreads();
+
+  if constexpr (METRICS) {
+    tail_metrics_phase2<TGT>(lg, reinterpret_cast<uint32_t*>(lg + C * TAIL_NPX), static_cast<const TGT*>(tgt), ms, b, h, w, C,
+                             oy0, ox0, yf, xf, sch, scw);
+    return;
+  }
 
   // ---- phase 2: bilinear x2 (align_corners=True) from shared memory; thread = 2 consecutive output pixels ----
   const int pr = threadIdx.x & 63, rq = threadIdx.x >> 6;
@@ -174,6 +193,67 @@ tail_fused_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __re
   }
 }
 
+// Phase 2 of the metrics epilogue: the thread / pixel mapping and the interpolation arithmetic of the argmax epilogue above
+// (so the predictions are the mask's, bit for bit), then log-sum-exp and the target logit over the same values.  No thread
+// returns early: the flush at the end is a CTA barrier.
+template <typename TGT>
+__device__ __forceinline__ void tail_metrics_phase2(const float* lg, uint32_t* hist, const TGT* __restrict__ tgt,
+                                                    const SegMetricsState& ms, int b, int h, int w, int C, int oy0, int ox0,
+                                                    int yf, int xf, float sch, float scw) {
+  const int Ho = 2 * h, Wo = 2 * w;
+  const int pr = threadIdx.x & 63, rq = threadIdx.x >> 6;
+  const int ox = ox0 + 2 * pr;
+  float loss = 0.f;
+  unsigned nvalid = 0, ninvalid = 0;
+  if (ox < Wo) {
+    float lx[2];
+    int d1, c0;
+    {
+      const float sx0 = scw * ox, sx1 = scw * (ox + 1);
+      const int x0 = (int)sx0, x1 = (int)sx1;
+      lx[0] = sx0 - x0; lx[1] = sx1 - x1;
+      d1 = x1 - x0;
+      c0 = x0 - xf;
+    }
+    const int ca = c0, cb = min(c0 + 1, TAIL_SC - 1), cc = min(c0 + 2, TAIL_SC - 1);
+    for (int ry = rq; ry < TAIL_TOH; ry += 4) {
+      const int oy = oy0 + ry;
+      if (oy >= Ho) break;
+      // the two targets of the pixel pair: one 16-byte (int64) or 2-byte (uint8) load; Wo and ox are even
+      long long t[2];
+      const long long o = ((long long)b * Ho + oy) * Wo + ox;
+      if constexpr (sizeof(TGT) == 8) {
+        const longlong2 tv = __ldg(reinterpret_cast<const longlong2*>(tgt + o));
+        t[0] = tv.x; t[1] = tv.y;
+      } else {
+        const unsigned short tv = __ldg(reinterpret_cast<const unsigned short*>(tgt + o));
+        t[0] = tv & 0xff; t[1] = tv >> 8;
+      }
+      const int tc[2] = {seg_target_class(t[0], C, ms.ignore_index), seg_target_class(t[1], C, ms.ignore_index)};
+      const float sy = sch * oy;
+      const int y0 = (int)sy;
+      const float ly = sy - y0, hy = 1.f - ly;
+      const int r0 = (y0 - yf) * TAIL_SC, r1 = r0 + (y0 < h - 1 ? TAIL_SC : 0);
+      SegPix px[2];
+      seg_pix_init(px[0]); seg_pix_init(px[1]);
+      for (int c = 0; c < C; ++c) {
+        const float* pl = lg + c * TAIL_NPX;
+        const float va = hy * pl[r0 + ca] + ly * pl[r1 + ca];
+        const float vb = hy * pl[r0 + cb] + ly * pl[r1 + cb];
+        const float vc = hy * pl[r0 + cc] + ly * pl[r1 + cc];
+        float v[2];
+        v[0] = (1.f - lx[0]) * va + lx[0] * vb;
+        v[1] = (1.f - lx[1]) * (d1 ? vb : va) + lx[1] * (d1 ? vc : vb);
+        seg_pix_step(px[0], v[0], c, tc[0]);
+        seg_pix_step(px[1], v[1], c, tc[1]);
+      }
+#pragma unroll
+      for (int e = 0; e < 2; ++e) seg_pix_finish(hist, px[e], t[e], tc[e], ms.ignore_index, C, loss, nvalid, ninvalid);
+    }
+  }
+  seg_flush(hist, C, loss, nvalid, ninvalid, hist + C * C, ms);
+}
+
 }  // namespace b200
 
 using namespace b200;
@@ -197,7 +277,8 @@ extern "C" int b200seg_tail_fused(const void* x, const void* w0, const float* b0
       attr = true;                                                                                                     \
     }                                                                                                                  \
     tail_fused_kernel<TO, AM><<<(unsigned)grid, 256, smem, st>>>((const bf16*)x, (const bf16*)w0, b0, (const bf16*)w3, b3, \
-                                                                 (TO*)out, mask, B, h, w, C, tiles_x, tiles_y);        \
+                                                                 (TO*)out, mask, B, h, w, C, tiles_x, tiles_y, nullptr, \
+                                                                 SegMetricsState{});                                   \
   }
   if (mask) TAIL_LAUNCH(float, true)
   else if (out_dtype == B200SEG_BF16) TAIL_LAUNCH(bf16, false)
@@ -205,4 +286,38 @@ extern "C" int b200seg_tail_fused(const void* x, const void* w0, const float* b0
   else return set_error(-1, "tail_fused: bad out dtype");
 #undef TAIL_LAUNCH
   return check_launch("tail_fused");
+}
+
+extern "C" int b200seg_tail_fused_metrics(const void* x, const void* w0, const float* b0, const void* w3, const float* b3,
+                                          const void* target, int target_dtype, long long ignore_index, int64_t* confusion,
+                                          int64_t* counts, double* loss_sum, int B, int h, int w, int C, b200seg_stream_t s) {
+  B200_REQUIRE(x && w0 && b0 && w3 && b3 && target && confusion && counts && loss_sum, "tail_fused_metrics: bad pointers");
+  B200_REQUIRE(C >= 1 && C <= 16 && B > 0 && h > 0 && w > 0, "tail_fused_metrics: bad shape (C=%d)", C);
+  B200_REQUIRE(target_dtype == B200SEG_I64 || target_dtype == B200SEG_U8, "tail_fused_metrics: target dtype must be int64 or uint8");
+  B200_REQUIRE((reinterpret_cast<uintptr_t>(target) & (target_dtype == B200SEG_I64 ? 15 : 1)) == 0,
+               "tail_fused_metrics: target must be %d-byte aligned", target_dtype == B200SEG_I64 ? 16 : 2);
+  const int tiles_x = (2 * w + TAIL_TOW - 1) / TAIL_TOW, tiles_y = (2 * h + TAIL_TOH - 1) / TAIL_TOH;
+  const long long grid = (long long)B * tiles_x * tiles_y;
+  B200_REQUIRE(grid < (1ll << 31), "tail_fused_metrics: too many tiles");
+  const size_t smem = ((size_t)C * TAIL_NPX + C * C + 24) * 4;
+  const SegMetricsState ms{reinterpret_cast<unsigned long long*>(confusion), reinterpret_cast<unsigned long long*>(counts),
+                           loss_sum, ignore_index};
+  cudaStream_t st = (cudaStream_t)s;
+  typedef __nv_bfloat16 bf16;
+#define TAIL_METRICS_LAUNCH(TGT)                                                                                       \
+  {                                                                                                                    \
+    static bool attr = false;                                                                                          \
+    if (!attr) {                                                                                                       \
+      cudaError_t e = cudaFuncSetAttribute(tail_fused_kernel<float, false, TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                           (16 * TAIL_NPX + 16 * 16 + 24) * 4);                                        \
+      if (e != cudaSuccess) return set_error((int)e, "tail_fused_metrics: cudaFuncSetAttribute: %s", cudaGetErrorString(e)); \
+      attr = true;                                                                                                     \
+    }                                                                                                                  \
+    tail_fused_kernel<float, false, TGT><<<(unsigned)grid, 256, smem, st>>>((const bf16*)x, (const bf16*)w0, b0,        \
+        (const bf16*)w3, b3, nullptr, nullptr, B, h, w, C, tiles_x, tiles_y, target, ms);                               \
+  }
+  if (target_dtype == B200SEG_I64) TAIL_METRICS_LAUNCH(int64_t)
+  else TAIL_METRICS_LAUNCH(uint8_t)
+#undef TAIL_METRICS_LAUNCH
+  return check_launch("tail_fused_metrics");
 }
