@@ -334,6 +334,27 @@ int b200seg_preprocess_u8(const uint8_t* frames, int B, int Hs, int Ws, void* ou
  * (0 = background in the reference). */
 int b200seg_remap_labels(const uint8_t* in, int64_t* out, const uint8_t* lut256, long long n, b200seg_stream_t s);
 
+/* ---------------------------------------------------------------------------------------------
+ * Object boxes from the class mask (inference.py:48-146, overlay_predictions), bit-equal to cv2 4.13 for every primitive:
+ * cv2.resize(mask [B,Hm,Wm] uint8, (W, H), INTER_NEAREST) -> per selected class classes[0..K-1] (1 <= K <= 16, distinct,
+ * in [0, 255]; a HOST array) the binary plane resized == class -> cv2.morphologyEx(MORPH_CLOSE, ones(close, close)) (close
+ * odd, 1..15; 1 = no close) -> cv2.connectedComponentsWithStats(connectivity=8).  Rows of the components with area >=
+ * min_area, per frame in (class position, cv2 label) order: stats int32 [B,max_objects,7] = class, label, left, top,
+ * width, height, area and centroid float64 [B,max_objects,2]; rows past the count are zero.  count int32 [B] = components
+ * with area >= min_area (may exceed max_objects: the rows past capacity are dropped).  labels (nullable) int32 [B,K,H,W]
+ * receives the cv2 label image of every plane.  workspace: device memory of at least b200seg_detect_workspace_bytes(B, K,
+ * H, W) bytes, 256-byte aligned.  Enqueues its kernels on s: no allocation, no synchronisation (capturable).
+ * --------------------------------------------------------------------------------------------- */
+int b200seg_detect_workspace_bytes(int B, int K, int H, int W, long long* bytes);
+int b200seg_detect_objects(const uint8_t* mask, int B, int Hm, int Wm, int H, int W, const int* classes, int K, int close,
+                           int min_area, int max_objects, void* workspace, long long workspace_bytes, int* count, int* stats,
+                           double* centroid, int* labels, b200seg_stream_t s);
+/* cv2.addWeighted(frames, alpha, palette[resized mask], beta, gamma) on uint8 BGR frames [B,H,W,3]: the mask [B,Hm,Wm] is
+ * resized INTER_NEAREST to HxW, palette is a device array of npal (0..256) BGR uint8 colours, mask values >= npal blend with
+ * black; out[B,H,W,3] = saturate(rint(fmaf(frame, alpha, fmaf(colour, beta, gamma)))). */
+int b200seg_overlay(const uint8_t* frames, const uint8_t* mask, int B, int Hm, int Wm, int H, int W, const uint8_t* palette,
+                    int npal, float alpha, float beta, float gamma, uint8_t* out, b200seg_stream_t s);
+
 #ifdef __cplusplus
 }
 #endif

@@ -13,7 +13,8 @@ from .preprocess import preprocess_image  # noqa: F401
 from .feed import DeviceFeeder, class_map_lut, remap_labels  # noqa: F401
 from .export import torch_graph  # noqa: F401
 from .metrics import SegmentationMetrics  # noqa: F401
+from .postprocess import Detections, detect_objects, overlay  # noqa: F401
 
 __all__ = ["MobileNetV2UNet", "UNet", "LightUNet", "CrossEntropyLoss", "Adam", "preprocess_image", "DeviceFeeder",
-           "class_map_lut", "remap_labels", "torch_graph", "SegmentationMetrics"]
+           "class_map_lut", "remap_labels", "torch_graph", "SegmentationMetrics", "detect_objects", "Detections", "overlay"]
 __version__ = "0.1.0"

@@ -83,6 +83,10 @@ _PROTOS = {
     "b200seg_grad_finalize_multi": [_vp, _vp, _vp, _i, _vp],
     "b200seg_grad_chunk": [],
     "b200seg_maxpool_bwd": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
+    # object boxes and overlay (postprocess.cu)
+    "b200seg_detect_workspace_bytes": [_i, _i, _i, _i, C.POINTER(_ll)],
+    "b200seg_detect_objects": [_vp, _i, _i, _i, _i, _i, C.POINTER(_i), _i, _i, _i, _i, _vp, _ll, _vp, _vp, _vp, _vp, _vp],
+    "b200seg_overlay": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i, _f, _f, _f, _vp, _vp],
 }
 EXPORTS = sorted(list(_PROTOS) + ["b200seg_last_error"])
 
