@@ -187,6 +187,34 @@ int b200seg_scale_unless_one(float* x, long long n, const float* s, b200seg_stre
 int b200seg_ce_count(const int64_t* target, float* counts, long long N, int C, long long ignore_index,
                      b200seg_stream_t s);
 
+/* nn.CrossEntropyLoss(weight, ignore_index, reduction, label_smoothing) with int64 or uint8 targets, fused forward and
+ * gradient.  A pixel is counted when its target t is in [0,C) and t != ignore_index (a uint8 label equals ignore_index only
+ * when ignore_index is in [0,255]).  For a counted pixel, with lse = logsumexp(z), w the class weights (all ones when
+ * weight is NULL), Wsum = sum_c w_c, eps = label_smoothing in [0,1]:
+ *   loss = (1-eps) w_t (lse - z_t) + eps/C sum_c w_c (lse - z_c)
+ *   grad = (1-eps) w_t (softmax - onehot_t) + eps/C (Wsum softmax - w)
+ * Other pixels: loss 0 and gradient 0, but a bad label (neither counted nor ignore_index) has a NaN loss.
+ *   logits NCHW f32 [B,C,H,W] (any C >= 1); target [B,H,W] of target_dtype B200SEG_I64 | B200SEG_U8; weight device f32 [C]
+ *   or NULL.
+ * b200seg_softmax_ce_ex: exactly one of
+ *   loss_sum f64[1] ('mean' / 'sum'): += sum of the pixel losses (caller zeroes); dlogits (or NULL) = grad / denom[0], or
+ *            grad alone when denom is NULL ('sum');
+ *   loss_map f32 [B,H,W] ('none'): the pixel losses; dlogits and denom must be NULL.
+ * b200seg_ce_count_ex: denom f64[2] += (sum of w_t over the counted pixels = the 'mean' divisor, number of bad labels);
+ *   caller zeroes.  N = B*H*W.
+ * b200seg_softmax_ce_ex_bwd: the backward of the loss map: dlogits = grad * gout (gout f32 [B,H,W]) in one pass over the
+ *   logits.
+ * 16-byte aligned logits, dlogits, loss_map, gout and target (uint8: 4-byte) with H*W % 4 == 0 and C <= 16 take the
+ * 4-pixel vector path; anything else the one-pixel kernels. */
+int b200seg_softmax_ce_ex(const float* logits, const void* target, int target_dtype, long long ignore_index,
+                          const float* weight, float label_smoothing, double* loss_sum, float* loss_map, float* dlogits,
+                          const double* denom, int B, int C, int H, int W, b200seg_stream_t s);
+int b200seg_ce_count_ex(const void* target, int target_dtype, long long ignore_index, const float* weight, double* denom,
+                        long long N, int C, b200seg_stream_t s);
+int b200seg_softmax_ce_ex_bwd(const float* logits, const void* target, int target_dtype, long long ignore_index,
+                              const float* weight, float label_smoothing, const float* gout, float* dlogits, int B, int C,
+                              int H, int W, b200seg_stream_t s);
+
 /* Any class count (outconv(in_ch, out_ch), unet.py:108-121, takes any out_ch; the fast kernels above hold <= 16
  * channels in registers): final_upsample to NCHW logits (mask == NULL) or to the uint8 argmax mask (out == NULL) from
  * NHWC logits with pixel pitch ldc >= C; its adjoint (dlogits NHWC [B,h,w,ldc], channels >= C zeroed); and the argmax

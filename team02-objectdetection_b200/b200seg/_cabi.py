@@ -47,6 +47,9 @@ _PROTOS = {
     "b200seg_scale_unless_one": [_vp, _ll, _vp, _vp],
     "b200seg_remap_labels": [_vp, _vp, _vp, _ll, _vp],
     "b200seg_ce_count": [_vp, _vp, _ll, _i, _ll, _vp],
+    "b200seg_softmax_ce_ex": [_vp, _vp, _i, _ll, _vp, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp],
+    "b200seg_ce_count_ex": [_vp, _i, _ll, _vp, _vp, _ll, _i, _vp],
+    "b200seg_softmax_ce_ex_bwd": [_vp, _vp, _i, _ll, _vp, _f, _vp, _vp, _i, _i, _i, _i, _vp],
     "b200seg_upsample2x_ac_generic": [_vp, _i, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp],
     "b200seg_final_bwd_generic": [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp],
     "b200seg_nhwc_argmax": [_vp, _i, _i, _vp, _ll, _i, _vp],

@@ -401,6 +401,65 @@ def softmax_ce(logits, target, want_grad: bool = True, grad_scale: Optional[floa
     return acc[0] / n, dl
 
 
+_TGT = {torch.int64: _cabi.I64, torch.uint8: _cabi.U8}
+
+
+def _ce_ex_args(logits, target, weight):
+    _cuda(logits, target, weight)
+    if logits.dtype != torch.float32 or logits.dim() != 4:
+        raise TypeError("softmax_ce_ex expects f32 NCHW logits")
+    if target.dtype not in _TGT:
+        raise TypeError(f"softmax_ce_ex: targets must be int64 or uint8, got {target.dtype}")
+    B, Cc, H, W = logits.shape
+    if tuple(target.shape) != (B, H, W):
+        raise ValueError(f"softmax_ce_ex: target shape {tuple(target.shape)} does not match logits {tuple(logits.shape)}")
+    if weight is not None:
+        if weight.dtype != torch.float32 or weight.dim() != 1 or weight.numel() != Cc:
+            raise ValueError(f"softmax_ce_ex: weight must be f32 [C={Cc}], got {weight.dtype} {tuple(weight.shape)}")
+        if weight.device != logits.device:
+            raise RuntimeError(f"softmax_ce_ex: weight on {weight.device}, logits on {logits.device}")
+    return B, Cc, H, W, _TGT[target.dtype]
+
+
+def softmax_ce_ex(logits, target, weight=None, ignore_index: int = IGNORE_INDEX, label_smoothing: float = 0.0,
+                  reduction: str = "mean", want_grad: bool = True):
+    """nn.CrossEntropyLoss(weight, ignore_index, reduction, label_smoothing) over NCHW f32 logits and int64 or uint8
+    targets (csrc/softmax_ce_ex.cu).  Returns (loss, dlogits or None).  'mean' / 'sum': a scalar, and dlogits of that
+    scalar from the same pass ('mean' divides by the weight sum of the counted targets, from b200seg_ce_count_ex).
+    'none': the f32 [B,H,W] loss map and no dlogits (softmax_ce_ex_backward gives them for an incoming gradient).  A
+    label outside [0,C) that is not ignore_index makes the loss NaN (per pixel for 'none')."""
+    B, Cc, H, W, tdt = _ce_ex_args(logits, target, weight)
+    if reduction == "none":
+        out = torch.empty((B, H, W), device=logits.device, dtype=torch.float32)
+        check(lib.b200seg_softmax_ce_ex(ptr(logits), ptr(target), tdt, ignore_index, ptr(weight), label_smoothing, None,
+                                        ptr(out), None, None, B, Cc, H, W, _stream()), "softmax_ce_ex")
+        return out, None
+    if reduction not in ("mean", "sum"):
+        raise ValueError(f"{reduction} is not a valid value for reduction")
+    acc = torch.zeros(3, device=logits.device, dtype=torch.float64)      # [loss sum, sum of w_t counted, bad labels]
+    dl = torch.empty_like(logits) if want_grad else None
+    if reduction == "mean":
+        check(lib.b200seg_ce_count_ex(ptr(target), tdt, ignore_index, ptr(weight), ptr(acc[1:]), B * H * W, Cc, _stream()),
+              "ce_count_ex")
+    check(lib.b200seg_softmax_ce_ex(ptr(logits), ptr(target), tdt, ignore_index, ptr(weight), label_smoothing, ptr(acc), None,
+                                    ptr(dl), ptr(acc[1:]) if reduction == "mean" else None, B, Cc, H, W, _stream()),
+          "softmax_ce_ex")
+    loss = acc[0] / acc[1] if reduction == "mean" else acc[0]           # 0/0 = NaN for an all-ignored batch, as torch
+    return loss.float(), dl
+
+
+def softmax_ce_ex_backward(logits, target, gout, weight=None, ignore_index: int = IGNORE_INDEX, label_smoothing: float = 0.0):
+    """d(sum(loss_map * gout)) / d(logits) of softmax_ce_ex(..., reduction='none'), one pass over the logits."""
+    B, Cc, H, W, tdt = _ce_ex_args(logits, target, weight)
+    _cuda(gout)
+    if gout.dtype != torch.float32 or tuple(gout.shape) != (B, H, W):
+        raise ValueError(f"softmax_ce_ex_backward: gout must be f32 {(B, H, W)}")
+    dl = torch.empty_like(logits)
+    check(lib.b200seg_softmax_ce_ex_bwd(ptr(logits), ptr(target), tdt, ignore_index, ptr(weight), label_smoothing, ptr(gout),
+                                        ptr(dl), B, Cc, H, W, _stream()), "softmax_ce_ex_bwd")
+    return dl
+
+
 def scale_unless_one(x, s):
     """x *= s (device scalar) in place; nothing is read or written when s == 1."""
     _cuda(x, s)

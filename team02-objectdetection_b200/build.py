@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "b200seg", "libb200seg.so")
-SOURCES = ["runtime.cu", "hbm_ops.cu", "conv_simt.cu", "conv_tc.cu", "conv_rs.cu", "softmax_ce.cu", "train_ops.cu", "conv_wgrad_tc.cu", "mbconv.cu", "adam.cu", "preprocess.cu", "generic_ops.cu", "tail_fused.cu", "stem_mb1.cu", "bn_cluster.cu", "seg_metrics.cu", "postprocess.cu"]
+SOURCES = ["runtime.cu", "hbm_ops.cu", "conv_simt.cu", "conv_tc.cu", "conv_rs.cu", "softmax_ce.cu", "train_ops.cu", "conv_wgrad_tc.cu", "mbconv.cu", "adam.cu", "preprocess.cu", "generic_ops.cu", "tail_fused.cu", "stem_mb1.cu", "bn_cluster.cu", "seg_metrics.cu", "postprocess.cu", "softmax_ce_ex.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC"]
