@@ -367,15 +367,26 @@ def run_forward(engine, x: torch.Tensor, mode: str, skip_out_step: bool = False)
     return env, saved
 
 
-def run_backward(engine, env, saved, mode: str, dout, ws: TrainWorkspace, g_src=None) -> None:
+def run_backward(engine, env, saved, mode: str, dout, ws: TrainWorkspace, g_src=None, keep: Optional[dict] = None) -> None:
     """Walk the schedule in reverse.  Parameter gradients are accumulated in ``ws`` staging; as soon as the last
     parameter of a gradient bucket is staged the bucket is finalized into the arena and (data parallel) its all-reduce
-    starts on the side stream while the walk continues."""
+    starts on the side stream while the walk continues.
+
+    ``keep`` (dict, as in ``engine.forward_eval``) receives a clone of every tensor gradient at the moment it is complete,
+    under ("d", tensor name), and of the dz each conv step feeds its weight- and data-gradient kernels, under
+    ("dz", step name).  Clones, because a gradient is handed on unchanged as the shortcut gradient of a block input."""
     sdt = torch.bfloat16 if mode == "bf16" else torch.float32
     tc = mode == "bf16" and (engine.dense_impl or "tc") == "tc"
     # g_src: the gradient of the output-layout step's INPUT, already computed by the caller outside the captured graph
     out_step = _out_step(engine) if g_src is not None else None
     g: Dict[str, torch.Tensor] = {"out": dout} if out_step is None else {out_step.src: g_src}
+
+    def pop(name):
+        t = g.pop(name)
+        if keep is not None:
+            keep[("d", name)] = t.clone()
+        return t
+
     ops.zero_pool.reset()
     ops.zero_pool32.reset()
     ws.begin_backward()
@@ -385,18 +396,18 @@ def run_backward(engine, env, saved, mode: str, dout, ws: TrainWorkspace, g_src=
         if s is out_step:
             continue
         if s.op in ("final", "to_nchw"):
-            g[s.src] = run_out_step_bwd(engine, s, env, g.pop(s.dst), sdt)
+            g[s.src] = run_out_step_bwd(engine, s, env, pop(s.dst), sdt)
         elif s.op == "upcat":
-            dcat = g.pop(s.dst)
+            dcat = pop(s.dst)
             cs = env[s.res].shape[-1]
             dskip, dx = ops.upcat_bwd(dcat, cs, g.get(s.res))
             g[s.res] = dskip
             assert s.src not in g
             g[s.src] = dx
         elif s.op == "pool":
-            g[s.src] = ops.maxpool_bwd(env[s.src], g.pop(s.dst), g.get(s.src))
+            g[s.src] = ops.maxpool_bwd(env[s.src], pop(s.dst), g.get(s.src))
         else:
-            da = g.pop(s.dst)
+            da = pop(s.dst)
             z = rec["z"]
             if s.bn is not None:
                 if s.op == "dense" and s.res:           # shortcut: the same gradient flows to the block input
@@ -406,6 +417,8 @@ def run_backward(engine, env, saved, mode: str, dout, ws: TrainWorkspace, g_src=
                 ws.done(s.bn.weight, s.bn.bias)
             else:
                 dz = da                                   # conv + bias only (the last 1x1 of outconv)
+            if keep is not None:
+                keep[("dz", s.name)] = dz.clone()
             w = s.conv.weight
             if s.conv.bias is not None:
                 ws.side(lambda: ops.colsum(dz, acc=ws.stage[id(s.conv.bias)]), dz)
