@@ -84,6 +84,15 @@ int b200seg_dwconv3x3_bf16w(const void* x, const void* w, const float* b, void* 
  *   flags: bit0 = store straight from registers instead of smem+TMA (debug / odd pitches) */
 int b200seg_conv_tc(const void* x, const void* w, const float* b, const void* res, void* y, int B, int H,
                     int W, int Cin, int Cout, int taps, int act, int flags, b200seg_stream_t s);
+/* Same convolution of cat([skip, x], channel) without materialising the concatenation (the first 3x3 conv of a decoder
+ * stage, unet.py:100-103 + 58): K chunks of the skip are loaded from skip, the rest from x, by TMA.
+ *   skip : NHWC bf16 [B,H,W,Cs], Cs % 8 == 0 (Cs = 0: skip unused, identical to b200seg_conv_tc)
+ *   x    : NHWC bf16 [B,H,W,Cu], Cu % 8 == 0
+ *   w    : bf16 [Cout][taps][Cs + Cu], the packing of the concatenated input
+ * Bit-identical to b200seg_conv_tc on the concatenated tensor when Cs % 64 == 0, and with Cs % 16 == 0 on maps narrower
+ * than 96 columns; otherwise the fp32 accumulation visits the K groups in another order. */
+int b200seg_conv_tc_cat(const void* skip, const void* x, const void* w, const float* b, const void* res, void* y, int B,
+                        int H, int W, int Cs, int Cu, int Cout, int taps, int act, int flags, b200seg_stream_t s);
 
 /* 3x3 convolution (pad 1, stride 1) with few output channels (Cout <= 32, or 65..80 for the data gradient of up4.conv.0:
  * N = 240, two accumulators = 480 TMEM columns) on wide maps as a ROW-STACKED implicit GEMM: the
@@ -94,6 +103,10 @@ int b200seg_conv_tc(const void* x, const void* w, const float* b, const void* re
 int b200seg_conv_rs_supported(int H, int W, int Cin, int Cout);
 int b200seg_conv_rs(const void* x, const void* w, const float* b, const void* res, void* y, int B, int H, int W, int Cin,
                     int Cout, int act, int flags, b200seg_stream_t s);
+/* Two-source input as in b200seg_conv_tc_cat: skip NHWC bf16 [B,H,W,Cs], x NHWC bf16 [B,H,W,Cu], w [Cout][9][Cs + Cu]. */
+int b200seg_conv_rs_cat_supported(int H, int W, int Cs, int Cu, int Cout);
+int b200seg_conv_rs_cat(const void* skip, const void* x, const void* w, const float* b, const void* res, void* y, int B,
+                        int H, int W, int Cs, int Cu, int Cout, int act, int flags, b200seg_stream_t s);
 
 /* Depthwise 3x3 on the tensor cores (bf16): the same TMA/tcgen05 pipeline as b200seg_conv_tc run over
  * 64-channel chunks with BLOCK-DIAGONAL weights, so the 9-tap stencil costs no CUDA-core FMAs or
@@ -112,7 +125,8 @@ int b200seg_conv_simt(const void* x, const float* w, const float* b, const void*
                       int B, int H, int W, int Cin, int Cout, int taps, int act, b200seg_stream_t s);
 
 /* up.forward (unet.py:100-103): y[..., :Cs] = skip ; y[..., Cs:] = bilinear_x2(x, align_corners=False).
- *   skip NHWC [B,2h,2w,Cs], x NHWC [B,h,w,Cu], y NHWC [B,2h,2w,Cs+Cu]. */
+ *   skip NHWC [B,2h,2w,Cs], x NHWC [B,h,w,Cu], y NHWC [B,2h,2w,Cs+Cu].  Cs = 0 (skip may be NULL): the upsample alone,
+ *   which b200seg_conv_tc_cat / b200seg_conv_rs_cat then read next to the skip tensor. */
 int b200seg_upsample2x_concat(const void* skip, const void* x, void* y, int dtype, int B, int h, int w,
                               int Cs, int Cu, b200seg_stream_t s);
 

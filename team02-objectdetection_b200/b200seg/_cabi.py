@@ -32,6 +32,9 @@ _PROTOS = {
     "b200seg_conv_tc": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     "b200seg_conv_rs_supported": [_i, _i, _i, _i],
     "b200seg_conv_rs": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp],
+    "b200seg_conv_tc_cat": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
+    "b200seg_conv_rs_cat_supported": [_i, _i, _i, _i, _i],
+    "b200seg_conv_rs_cat": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     "b200seg_dwconv3x3_tc": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp],
     "b200seg_mbconv": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     "b200seg_conv_simt": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],

@@ -29,7 +29,7 @@ from .ops import ACT_NONE, ACT_RELU, ACT_RELU6
 
 @dataclass
 class Step:
-    op: str                      # stem | dw | dense | upcat | pool | final | to_nchw
+    op: str                      # stem | dw | dense | upcat | upsample | pool | final | to_nchw
     name: str                    # module path (debug / profiling labels)
     src: str
     dst: str
@@ -41,6 +41,7 @@ class Step:
     res: Optional[str] = None    # residual source (dense) / skip source (upcat)
     pad_cout: int = 0            # pad output channels (logits 10 -> 16)
     parts: Optional[tuple] = None   # op == "mbconv": the (expand, depthwise, project) steps it replaces
+    skip: Optional[str] = None   # dense on two sources: the input is cat([skip, src], channel), never materialised
 
 
 def _double_conv_steps(prefix: str, dc, src: str, dst: str) -> List[Step]:
@@ -329,8 +330,30 @@ class Engine:
                     and tuple(out[-3].conv.weight.shape[:2]) == (16, 32) and out[-2].conv.weight.shape[1] == 16):
                 c0, c3, fin = out[-3], out[-2], out[-1]
                 out = out[:-3] + [Step("tail", "outc+final_upsample", c0.src, fin.dst, parts=(c0, c3, fin))]
-            self._eval_sched[key] = out
+            self._eval_sched[key] = self._split_upcat(out)
         return self._eval_sched[key]
+
+    @staticmethod
+    def _split_upcat(steps: List[Step]) -> List[Step]:
+        """Decoder stages without a concat buffer: an upsample+concat whose only reader is a 3x3 dense conv becomes the
+        upsample alone, and the conv reads cat([skip, upsampled]) from the two tensors (conv_tc / conv_rs two-source A
+        operand).  The skip is no longer copied into the concat buffer and read back: 209.6 MB less traffic per
+        MobileNetV2UNet step at B = 64, 256 x 512.  Step names stay, so profiles line up with the unsplit schedule."""
+        import dataclasses
+        out = list(steps)
+        for i, st in enumerate(steps):
+            if st.op != "upcat" or st.res is None:
+                continue
+            users = [j for j, t in enumerate(steps) if st.dst in (t.src, t.res, t.skip)]
+            if len(users) != 1:
+                continue
+            c = steps[users[0]]
+            if c.op != "dense" or c.taps != 9 or c.src != st.dst or c.res == st.dst or c.skip is not None:
+                continue
+            up = st.dst + ".u"
+            out[i] = Step("upsample", st.name, st.src, up)
+            out[users[0]] = dataclasses.replace(c, src=up, skip=st.res)
+        return out
 
     # ------------------------------------------------------------------ helpers
     def _mode(self, x: torch.Tensor) -> str:
@@ -381,8 +404,10 @@ class Engine:
             p = pk[s.name]
             res = env[s.res] if s.res else None
             if dense_impl == "tc":
-                env[s.dst] = ops.conv_tc(env[s.src], p["w"], p["b"], s.taps, s.act, res, flags=self.tc_flags)
+                env[s.dst] = ops.conv_tc(env[s.src], p["w"], p["b"], s.taps, s.act, res, flags=self.tc_flags,
+                                         skip=env[s.skip] if s.skip else None)
             else:
+                assert s.skip is None, "two-source steps are scheduled on the tensor-core path only"
                 env[s.dst] = ops.conv_simt(env[s.src], p["w"], p["b"], s.taps, s.act, res)
         elif s.op == "stem_mb1":
             p0, p1, p2 = (pk[q.name] for q in s.parts)
@@ -402,6 +427,8 @@ class Engine:
             env[s.dst] = ops.tail_fused(env[s.src], p0["w"], p0["b64"], p3["w"], p3["b64"], self.out_ch, out_dtype, want_mask, out=out)
         elif s.op == "upcat":
             env[s.dst] = ops.upsample2x_concat(env[s.res], env[s.src])
+        elif s.op == "upsample":
+            env[s.dst] = ops.upsample2x_concat(None, env[s.src])
         elif s.op == "pool":
             env[s.dst] = ops.maxpool2x2(env[s.src])
         elif s.op in ("final", "to_nchw") and metrics is not None:
@@ -559,6 +586,8 @@ class Engine:
             return nbytes, flops
         if s.res:
             nbytes += env[s.res].numel() * env[s.res].element_size()
+        if s.skip:
+            nbytes += env[s.skip].numel() * env[s.skip].element_size()
         if s.conv is not None:
             p = pk[s.name]
             nbytes += p["w"].numel() * p["w"].element_size() + p["b"].numel() * 4
@@ -569,7 +598,8 @@ class Engine:
                 flops = 2 * out.numel() * 27
             else:
                 cout = s.conv.weight.shape[0]                      # real (unpadded) output channels
-                flops = 2 * (out.numel() // out.shape[-1]) * cout * s.taps * env[s.src].shape[-1]
+                cin = env[s.src].shape[-1] + (env[s.skip].shape[-1] if s.skip else 0)
+                flops = 2 * (out.numel() // out.shape[-1]) * cout * s.taps * cin
         return nbytes, flops
 
     # ------------------------------------------------------------------ dispatch

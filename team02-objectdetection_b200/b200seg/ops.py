@@ -142,23 +142,42 @@ USE_CONV_RS = True       # 3x3 convs with <= 32 output channels on wide maps go 
 CONV_RS_FLAGS = 0        # tuning flags of b200seg_conv_rs (tools only)
 
 
-def conv_rs(x, w, b, act: int, res=None, out=None, flags: int = 0):
-    """Row-stacked 3x3 tensor-core conv for few output channels: same operands/results as conv_tc(taps=9)."""
-    _cuda(x, w, b, res)
+def _skip_channels(skip, x, what: str) -> int:
+    """Channels of the skip half of a two-source input cat([skip, x], channel) (0 without a skip)."""
+    if skip is None:
+        return 0
+    if skip.dtype != x.dtype or skip.shape[:3] != x.shape[:3] or not skip.is_contiguous():
+        raise ValueError(f"{what}: skip {tuple(skip.shape)} {skip.dtype} vs x {tuple(x.shape)} {x.dtype}")
+    return skip.shape[3]
+
+
+def conv_rs(x, w, b, act: int, res=None, out=None, flags: int = 0, skip=None):
+    """Row-stacked 3x3 tensor-core conv for few output channels: same operands/results as conv_tc(taps=9).
+    ``skip``: the input is cat([skip, x], channel), read from the two tensors (see conv_tc)."""
+    _cuda(x, w, b, res, skip)
     if x.dtype != torch.bfloat16 or w.dtype != torch.bfloat16:
         raise TypeError("conv_rs is bf16-only")
-    B, H, W, Cin = x.shape
+    B, H, W, Cu = x.shape
+    Cs = _skip_channels(skip, x, "conv_rs")
     Cout = w.shape[0]
-    if w.shape[1] != 9 * Cin:
-        raise ValueError(f"conv_rs: weight {tuple(w.shape)} does not match Cin={Cin}")
+    if w.shape[1] != 9 * (Cs + Cu):
+        raise ValueError(f"conv_rs: weight {tuple(w.shape)} does not match Cin={Cs + Cu}")
     if out is None:
         out = torch.empty((B, H, W, Cout), device=x.device, dtype=torch.bfloat16)
-    check(lib.b200seg_conv_rs(ptr(x), ptr(w), ptr(b), ptr(res), ptr(out), B, H, W, Cin, Cout, act, flags, _stream()), "conv_rs")
+    if skip is None:
+        check(lib.b200seg_conv_rs(ptr(x), ptr(w), ptr(b), ptr(res), ptr(out), B, H, W, Cu, Cout, act, flags, _stream()), "conv_rs")
+    else:
+        check(lib.b200seg_conv_rs_cat(ptr(skip), ptr(x), ptr(w), ptr(b), ptr(res), ptr(out), B, H, W, Cs, Cu, Cout, act, flags,
+                                      _stream()), "conv_rs_cat")
     return out
 
 
-def conv_tc(x, w, b, taps: int, act: int, res=None, out=None, flags: int = 0):
-    """Tensor-core conv. x NHWC bf16 [B,H,W,Cin]; w bf16 [Cout, taps*Cin]; b f32 [Cout]."""
+def conv_tc(x, w, b, taps: int, act: int, res=None, out=None, flags: int = 0, skip=None):
+    """Tensor-core conv. x NHWC bf16 [B,H,W,Cin]; w bf16 [Cout, taps*Cin]; b f32 [Cout].
+    ``skip`` NHWC bf16 [B,H,W,Cs]: the input is cat([skip, x], channel) and w is packed for Cin = Cs + Cu; the kernel loads
+    each 64-channel K chunk from the tensor it lies in, so the concatenation is never written."""
+    if skip is not None:
+        return _conv_tc_cat(skip, x, w, b, taps, act, res, out, flags)
     _cuda(x, w, b, res)
     if x.dtype != torch.bfloat16 or w.dtype != torch.bfloat16:
         raise TypeError("conv_tc is bf16-only")
@@ -175,6 +194,27 @@ def conv_tc(x, w, b, taps: int, act: int, res=None, out=None, flags: int = 0):
         out = torch.empty((B, H, W, Cout), device=x.device, dtype=torch.bfloat16)
     check(lib.b200seg_conv_tc(ptr(x), ptr(w), ptr(b), ptr(res), ptr(out), B, H, W, Cin, Cout, taps, act, flags,
                               _stream()), "conv_tc")
+    return out
+
+
+def _conv_tc_cat(skip, x, w, b, taps: int, act: int, res, out, flags: int):
+    """conv_tc on cat([skip, x], channel) read from the two tensors (kept apart from the one-source path, which the
+    training step calls a few hundred times per step)."""
+    _cuda(x, w, b, res, skip)
+    if x.dtype != torch.bfloat16 or w.dtype != torch.bfloat16:
+        raise TypeError("conv_tc is bf16-only")
+    B, H, W, Cu = x.shape
+    Cs = _skip_channels(skip, x, "conv_tc")
+    Cout = w.shape[0]
+    if w.shape[1] != taps * (Cs + Cu):
+        raise ValueError(f"conv_tc: weight {tuple(w.shape)} does not match taps={taps} Cin={Cs + Cu}")
+    if (taps == 9 and USE_CONV_RS and flags == 0 and lib.b200seg_conv_rs_cat_supported(H, W, Cs, Cu, Cout)
+            and (Cout <= 32 or res is None)):
+        return conv_rs(x, w, b, act, res, out, CONV_RS_FLAGS, skip=skip)
+    if out is None:
+        out = torch.empty((B, H, W, Cout), device=x.device, dtype=torch.bfloat16)
+    check(lib.b200seg_conv_tc_cat(ptr(skip), ptr(x), ptr(w), ptr(b), ptr(res), ptr(out), B, H, W, Cs, Cu, Cout, taps, act,
+                                  flags, _stream()), "conv_tc_cat")
     return out
 
 
@@ -228,11 +268,11 @@ def mbconv(x, w_exp, b_exp, w_dw, b_dw, w_proj, b_proj, stride: int, residual: b
 
 
 def upsample2x_concat(skip, x, out=None):
-    """cat([skip, bilinear_x2(x, align_corners=False)], channel) in NHWC."""
+    """cat([skip, bilinear_x2(x, align_corners=False)], channel) in NHWC; skip None: the upsample alone."""
     _cuda(skip, x)
     B, h, w, Cu = x.shape
-    Cs = skip.shape[3]
-    if skip.shape[:3] != (B, 2 * h, 2 * w) or skip.dtype != x.dtype:
+    Cs = 0 if skip is None else skip.shape[3]
+    if skip is not None and (skip.shape[:3] != (B, 2 * h, 2 * w) or skip.dtype != x.dtype):
         raise ValueError(f"upsample2x_concat: skip {tuple(skip.shape)} vs x {tuple(x.shape)}")
     if out is None:
         out = torch.empty((B, 2 * h, 2 * w, Cs + Cu), device=x.device, dtype=x.dtype)

@@ -18,6 +18,9 @@
 // input row and 64-channel chunk, borders = TMA zero fill), warp 1 TMEM owner + MMA issuer (weights resident in shared
 // memory, 3 x 3 x chunks tiles of [3*CN][64]), warps 2..5 epilogue.  Two TMEM accumulators: the MMAs of row r+1 overlap the
 // epilogue of row r.
+//
+// Two-source input (b200seg_conv_rs_cat): cat([S, U], channel) read from the two dense tensors as in conv_tc -- chunks
+// 0 .. ks-1 from S, the rest from U, weight columns at Cs + 64(c - ks) for a U chunk (see conv_tc.cu).
 #include "common.cuh"
 
 namespace b200 {
@@ -29,7 +32,8 @@ struct ConvRsArgs {
   int Cin, Cout;
   int W, H, B;
   int BW, tiles_w;
-  int k_chunks, stages;
+  int k_chunks, stages;   // k_chunks = ceil(Cs / 64) + ceil((Cin - Cs) / 64)
+  int Cs, ks;             // two-source input: channels of S and its chunk count; 0 = one source
   int act;
   long long total_rows;   // B * tiles_w * H
 };
@@ -51,12 +55,15 @@ __device__ __forceinline__ void rs_walk(long long g0, long long g1, int H, F&& f
   }
 }
 
-template <int CN>
+// CAT: two-source input (Cs > 0); the one-source instantiation carries no per-chunk source selection
+template <int CN, bool CAT>
 __global__ void __launch_bounds__(RS_THREADS, CN <= 32 ? 2 : 1)
-conv_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const ConvRsArgs a) {
+conv_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+               const __grid_constant__ CUtensorMap tmS, const ConvRsArgs a) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int ks = CAT ? a.ks : 0, Cs = CAT ? a.Cs : 0;
   constexpr int NACC = 3 * CN;                    // accumulator columns per input row
   constexpr int B_TILE = NACC * 128;              // one (chunk, kw) weight tile: [3*CN rows][64 k] bf16
 
@@ -73,6 +80,7 @@ conv_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
+    if (CAT) tma_prefetch_desc(&tmS);
     for (int i = 0; i < a.stages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 128); }
     mbar_init(b_full, 1);
@@ -97,7 +105,8 @@ conv_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       for (int c = 0; c < a.k_chunks; ++c)
         for (int kw = 0; kw < 3; ++kw)
           for (int kh = 0; kh < 3; ++kh)          // rows [kh*CN, +CN) of tile (c, kw) <- W[:, tap kh*3+kw, chunk c]
-            tma_load_3d(sB + (c * 3 + kw) * B_TILE + kh * CN * 128, &tmB, b_full, c * 64, kh * 3 + kw, 0);
+            tma_load_3d(sB + (c * 3 + kw) * B_TILE + kh * CN * 128, &tmB, b_full, CAT && c < ks ? c * 64 : Cs + (c - ks) * 64,
+                        kh * 3 + kw, 0);
     }
     int s = 0;
     uint32_t ph = 0;
@@ -108,7 +117,8 @@ conv_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         mbar_wait(&empty[s], ph ^ 1u, 1);
         if (lane == 0) {
           mbar_arrive_expect_tx(&full[s], 130u * 128u);
-          tma_load_4d(sA + s * RS_HALO_BYTES, &tmA, &full[s], c * 64, w0 - 1, r, bb);
+          const bool sk = CAT && c < ks;
+          tma_load_4d(sA + s * RS_HALO_BYTES, sk ? &tmS : &tmA, &full[s], sk ? c * 64 : (c - ks) * 64, w0 - 1, r, bb);
         }
         __syncwarp();
         if (++s == a.stages) { s = 0; ph ^= 1u; }
@@ -133,7 +143,8 @@ conv_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const uint32_t tacc = tmem_base + (uint32_t)(ab * NACC);
       uint32_t first = 0;
       for (int c = 0; c < a.k_chunks; ++c) {
-        const int ksteps = (min(64, a.Cin - c * 64) + 15) >> 4;
+        const int krem = CAT && c < ks ? Cs - c * 64 : a.Cin - Cs - (c - ks) * 64;   // channels left in the chunk's source
+        const int ksteps = (min(64, krem) + 15) >> 4;
         const uint32_t a_lo = a_lo0 + (uint32_t)s * (RS_HALO_BYTES >> 4);
         mbar_wait(&full[s], ph, 2);
         tc_fence_after();
@@ -239,8 +250,9 @@ conv_rs_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
 }
 
-template <int CN>
-static int launch_conv_rs(const CUtensorMap& tmA, const CUtensorMap& tmB, ConvRsArgs a, int flags, cudaStream_t stream) {
+template <int CN, bool CAT>
+static int launch_conv_rs(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmS, ConvRsArgs a, int flags,
+                          cudaStream_t stream) {
   const int b_all = a.k_chunks * 3 * (3 * CN * 128);
   const int fixed = b_all + CN * 4 + 256 + 1024 /*align slack*/;
   const int tmem_cols = 2 * 3 * CN <= 256 ? 256 : 512;
@@ -257,14 +269,14 @@ static int launch_conv_rs(const CUtensorMap& tmA, const CUtensorMap& tmB, ConvRs
   const int smem = fixed + stages * RS_HALO_BYTES;
   static bool attr = false;
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(conv_rs_kernel<CN>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(conv_rs_kernel<CN, CAT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return set_error((int)e, "conv_rs: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     attr = true;
   }
   long long grid = (long long)sm_count() * per_sm;
   if ((flags >> 8) & 0xff) grid = (long long)((flags >> 8) & 0xff) * 4;
   if (grid > a.total_rows) grid = a.total_rows;
-  conv_rs_kernel<CN><<<(unsigned)grid, RS_THREADS, (size_t)smem, stream>>>(tmA, tmB, a);
+  conv_rs_kernel<CN, CAT><<<(unsigned)grid, RS_THREADS, (size_t)smem, stream>>>(tmA, tmB, tmS, a);
   return check_launch("conv_rs");
 }
 
@@ -272,40 +284,49 @@ static int launch_conv_rs(const CUtensorMap& tmA, const CUtensorMap& tmB, ConvRs
 
 using namespace b200;
 
-// 1 if b200seg_conv_rs supports the shape (the engine asks before choosing it over b200seg_conv_tc)
-extern "C" int b200seg_conv_rs_supported(int H, int W, int Cin, int Cout) {
+static int rs_supported(int H, int W, int Cs, int Cin, int Cout) {
   const int cn = (Cout + 15) & ~15;
-  const int k_chunks = (Cin + 63) / 64;
+  const int k_chunks = (Cs + 63) / 64 + (Cin - Cs + 63) / 64;
   // cn = 80: the data gradient of up4.conv.0 (32 -> 80 channels): N = 240, two accumulators = 480 TMEM columns, the
   // epilogue's two running rows take 160 registers (one CTA per SM, 255 registers per thread)
   return (cn == 16 || cn == 32 || cn == 80) && W >= 96 && H >= 3 && Cin % 8 == 0 && Cout % 8 == 0 &&
          k_chunks * 3 * (3 * cn * 128) <= 120 * 1024;
 }
 
+// 1 if b200seg_conv_rs supports the shape (the engine asks before choosing it over b200seg_conv_tc)
+extern "C" int b200seg_conv_rs_supported(int H, int W, int Cin, int Cout) { return rs_supported(H, W, 0, Cin, Cout); }
+
+// the same for b200seg_conv_rs_cat (skip S with Cs channels + U with Cu channels)
+extern "C" int b200seg_conv_rs_cat_supported(int H, int W, int Cs, int Cu, int Cout) {
+  return Cs >= 0 && Cs % 8 == 0 && Cu > 0 && rs_supported(H, W, Cs, Cs + Cu, Cout);
+}
+
 // 3x3, pad 1, stride 1, bf16 NHWC, few output channels (see b200seg_conv_rs_supported).  Same operands and results as
 // b200seg_conv_tc(taps = 9): w bf16 [Cout][9][Cin], b f32 [Cout] or NULL, res added after the activation.
 // flags: bits 8..15 grid/4, bits 16..19 max ring stages, bits 20..21 CTAs per SM (0 = auto).
-extern "C" int b200seg_conv_rs(const void* x, const void* w, const float* bias, const void* res, void* y, int B, int H,
-                               int W, int Cin, int Cout, int act, int flags, b200seg_stream_t s) {
-  B200_REQUIRE(x && w && y && B > 0, "conv_rs: bad arguments");
-  B200_REQUIRE(b200seg_conv_rs_supported(H, W, Cin, Cout), "conv_rs: unsupported shape H=%d W=%d Cin=%d Cout=%d", H, W, Cin, Cout);
+static int conv_rs_run(const void* skip, int Cs, const void* x, const void* w, const float* bias, const void* res, void* y,
+                       int B, int H, int W, int Cin, int Cout, int act, int flags, cudaStream_t stream) {
+  const int Cu = Cin - Cs;
   ConvRsArgs a;
   a.bias = bias; a.res = res; a.y = y;
   a.Cin = Cin; a.Cout = Cout; a.W = W; a.H = H; a.B = B;
   a.BW = W < 128 ? W : 128;
   a.tiles_w = (W + a.BW - 1) / a.BW;
-  a.k_chunks = (Cin + 63) / 64;
+  a.k_chunks = (Cs + 63) / 64 + (Cu + 63) / 64;
+  a.Cs = Cs; a.ks = (Cs + 63) / 64;
   a.act = act;
   a.total_rows = (long long)B * a.tiles_w * H;
   const int cn = (Cout + 15) & ~15;
-  CUtensorMap tmA, tmB;
-  {
-    uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)W, (uint64_t)H, (uint64_t)B};
-    uint64_t str[3] = {(uint64_t)Cin * 2, (uint64_t)Cin * 2 * W, (uint64_t)Cin * 2 * W * H};
+  CUtensorMap tmA, tmB, tmS;
+  for (int src = 0; src < (Cs ? 2 : 1); ++src) {
+    const uint64_t c = (uint64_t)(src ? Cs : Cu);
+    uint64_t dims[4] = {c, (uint64_t)W, (uint64_t)H, (uint64_t)B};
+    uint64_t str[3] = {c * 2, c * 2 * W, c * 2 * W * H};
     uint32_t box[4] = {64, 130, 1, 1};
-    int rc = make_tmap_bf16(&tmA, x, 4, dims, str, box, 1, nullptr);
+    int rc = make_tmap_bf16(src ? &tmS : &tmA, src ? skip : x, 4, dims, str, box, 1, nullptr);
     if (rc) return rc;
   }
+  if (!Cs) tmS = tmA;
   {
     uint64_t dims[3] = {(uint64_t)Cin, 9, (uint64_t)Cout};
     uint64_t str[2] = {(uint64_t)Cin * 2, (uint64_t)Cin * 2 * 9};
@@ -313,7 +334,29 @@ extern "C" int b200seg_conv_rs(const void* x, const void* w, const float* bias, 
     int rc = make_tmap_bf16(&tmB, w, 3, dims, str, box, 1, nullptr);
     if (rc) return rc;
   }
-  if (cn == 16) return launch_conv_rs<16>(tmA, tmB, a, flags, (cudaStream_t)s);
-  if (cn == 80) return launch_conv_rs<80>(tmA, tmB, a, flags, (cudaStream_t)s);
-  return launch_conv_rs<32>(tmA, tmB, a, flags, (cudaStream_t)s);
+  if (Cs) {
+    if (cn == 16) return launch_conv_rs<16, true>(tmA, tmB, tmS, a, flags, stream);
+    if (cn == 80) return launch_conv_rs<80, true>(tmA, tmB, tmS, a, flags, stream);
+    return launch_conv_rs<32, true>(tmA, tmB, tmS, a, flags, stream);
+  }
+  if (cn == 16) return launch_conv_rs<16, false>(tmA, tmB, tmS, a, flags, stream);
+  if (cn == 80) return launch_conv_rs<80, false>(tmA, tmB, tmS, a, flags, stream);
+  return launch_conv_rs<32, false>(tmA, tmB, tmS, a, flags, stream);
+}
+
+extern "C" int b200seg_conv_rs(const void* x, const void* w, const float* bias, const void* res, void* y, int B, int H,
+                               int W, int Cin, int Cout, int act, int flags, b200seg_stream_t s) {
+  B200_REQUIRE(x && w && y && B > 0, "conv_rs: bad arguments");
+  B200_REQUIRE(b200seg_conv_rs_supported(H, W, Cin, Cout), "conv_rs: unsupported shape H=%d W=%d Cin=%d Cout=%d", H, W, Cin, Cout);
+  return conv_rs_run(nullptr, 0, x, w, bias, res, y, B, H, W, Cin, Cout, act, flags, (cudaStream_t)s);
+}
+
+// two-source input: cat([skip [B,H,W,Cs], x [B,H,W,Cu]], channel), w bf16 [Cout][9][Cs + Cu]
+extern "C" int b200seg_conv_rs_cat(const void* skip, const void* x, const void* w, const float* bias, const void* res,
+                                   void* y, int B, int H, int W, int Cs, int Cu, int Cout, int act, int flags,
+                                   b200seg_stream_t s) {
+  B200_REQUIRE(x && w && y && B > 0 && (skip || !Cs), "conv_rs_cat: bad arguments");
+  B200_REQUIRE(b200seg_conv_rs_cat_supported(H, W, Cs, Cu, Cout), "conv_rs_cat: unsupported shape H=%d W=%d Cs=%d Cu=%d Cout=%d",
+               H, W, Cs, Cu, Cout);
+  return conv_rs_run(skip, Cs, x, w, bias, res, y, B, H, W, Cs + Cu, Cout, act, flags, (cudaStream_t)s);
 }

@@ -19,6 +19,13 @@
 // B operand (weights bf16 [Cout][taps][Cin]): 3-D map, box {64,1,N}; when all taps/chunks of the N
 // tile fit in shared memory they are loaded once per CTA ("resident") instead of once per tile.
 //
+// Two-source A (the decoder's first 3x3 conv of an up stage): the input is cat([S, U], channel) with S
+// [B][H][W][Cs] and U [B][H][W][Cu] kept as two dense tensors.  K chunks 0 .. ks-1 (ks = ceil(Cs/64)) load
+// from a map over S at channel 64c, the rest from the map over U at channel 64(c-ks); the weight box of a U
+// chunk starts at channel Cs + 64(c-ks).  In a narrow skip chunk the weight columns past Cs belong to U, but
+// they meet S's out-of-bounds zero fill and add exact zeros; the chunk issues ceil((Cs-64c)/16) k-steps, so
+// the issued MMAs are those of the concatenated tensor.  Cs = 0 is the single-tensor path.
+//
 // Epilogue: TMEM -> registers (tcgen05.ld 32x32b.x16, double-buffered) -> +bias -> ReLU/ReLU6 -> +residual
 // -> bf16 -> one 256-bit global store per 16 channels (thread = pixel, so each store is a full 32-byte
 // sector of that pixel's NHWC row).  An alternative epilogue (flag bit0) goes through a 128B-swizzled
@@ -40,7 +47,8 @@ struct ConvTcArgs {
   int BW, BH;        // M tile = BH rows x BW columns of pixels, BW*BH <= 128
   int tiles_w, tiles_h;
   int block_n, n_tiles;
-  int k_chunks;      // ceil(Cin / 64)
+  int k_chunks;      // ceil(Cs / 64) + ceil((Cin - Cs) / 64)
+  int Cs, ks;        // two-source A: channels of S and its chunk count ceil(Cs / 64); 0 = one source
   int stages;
   int act;
   int tma_store;     // epilogue: 0 = 256-bit stores straight from registers, 1 = smem staging + TMA store
@@ -68,14 +76,16 @@ __device__ __forceinline__ uint64_t umma_desc_k128_off(uint32_t smem_addr) {
   return umma_desc_k128(smem_addr) | ((uint64_t)((smem_addr >> 7) & 7u) << 49);
 }
 
-template <int MPAIR>
+// CAT: two-source A (Cs > 0).  The one-source instantiation carries none of the per-chunk source selection.
+template <int MPAIR, bool CAT>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const __grid_constant__ CUtensorMap tmC, const ConvTcArgs a) {
+               const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmS, const ConvTcArgs a) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int ks = CAT ? a.ks : 0, Cs = CAT ? a.Cs : 0;
   const int n_boxes = (a.block_n + 63) >> 6;
   const int kb_per_tile = a.halo ? a.k_chunks * 3 : a.k_chunks * a.taps;
   const int b_tiles_resident = a.taps * a.k_chunks;
@@ -97,6 +107,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
+    if (CAT) tma_prefetch_desc(&tmS);
     if (a.tma_store) tma_prefetch_desc(&tmC);
     for (int i = 0; i < a.stages; ++i) {
       mbar_init(&full[i], 1);
@@ -125,7 +136,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       mbar_arrive_expect_tx(b_full, (uint32_t)(b_tiles_resident * b_tile_bytes));
       for (int t = 0; t < a.taps; ++t)
         for (int c = 0; c < a.k_chunks; ++c)
-          tma_load_3d(sB + (t * a.k_chunks + c) * b_tile_bytes, &tmB, b_full, c * 64, t, 0);
+          tma_load_3d(sB + (t * a.k_chunks + c) * b_tile_bytes, &tmB, b_full, CAT && c < ks ? c * 64 : Cs + (c - ks) * 64, t, 0);
     }
     pdl_wait();         // weights are static; activations come from the previous kernel
     int s = 0;
@@ -153,25 +164,31 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (a.halo) {
               const int chunk = o, dh = i;
               const int ach = a.dw ? n_tile : chunk;           // channel chunk of the activations
+              const bool sk = CAT && ach < ks;                 // chunk of the skip source
+              const CUtensorMap* tmX = sk ? &tmS : &tmA;
+              const int xc = sk ? ach * 64 : (ach - ks) * 64, wc = sk ? chunk * 64 : Cs + (chunk - ks) * 64;
 #pragma unroll
               for (int j = 0; j < MPAIR; ++j)
-                tma_load_4d(sA + s * a_stride + j * a.a_stage_bytes, &tmA, &full[s], ach * 64, w0v[j] - 1,
+                tma_load_4d(sA + s * a_stride + j * a.a_stage_bytes, tmX, &full[s], xc, w0v[j] - 1,
                             h0v[j] + dh - 1, bbv[j]);
               if (!a.b_resident)
                 for (int dw = 0; dw < 3; ++dw)
-                  tma_load_3d(sB + s * a.b_stage_bytes + dw * b_tile_bytes, &tmB, &full[s], a.dw ? 0 : chunk * 64,
+                  tma_load_3d(sB + s * a.b_stage_bytes + dw * b_tile_bytes, &tmB, &full[s], a.dw ? 0 : wc,
                               dh * 3 + dw, n0);
             } else {
               const int tap = o, chunk = i;
               const int ach = a.dw ? n_tile : chunk;
+              const bool sk = CAT && ach < ks;
+              const CUtensorMap* tmX = sk ? &tmS : &tmA;
+              const int xc = sk ? ach * 64 : (ach - ks) * 64, wc = sk ? chunk * 64 : Cs + (chunk - ks) * 64;
               int dw = 0, dh = 0;
               if (a.taps == 9) { dh = tap / 3 - 1; dw = tap - (dh + 1) * 3 - 1; }
 #pragma unroll
               for (int j = 0; j < MPAIR; ++j)
-                tma_load_4d(sA + s * a_stride + j * a.a_stage_bytes, &tmA, &full[s], ach * 64, w0v[j] * a.stride + dw,
+                tma_load_4d(sA + s * a_stride + j * a.a_stage_bytes, tmX, &full[s], xc, w0v[j] * a.stride + dw,
                             h0v[j] * a.stride + dh, bbv[j]);
               if (!a.b_resident)
-                tma_load_3d(sB + s * a.b_stage_bytes, &tmB, &full[s], a.dw ? 0 : chunk * 64, tap, n0);
+                tma_load_3d(sB + s * a.b_stage_bytes, &tmB, &full[s], a.dw ? 0 : wc, tap, n0);
             }
           }
           __syncwarp();
@@ -208,7 +225,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       for (int o = 0; o < n_outer; ++o) {
         for (int i = 0; i < n_inner; ++i) {
           const int chunk = a.halo ? o : i;
-          const int ksteps = (min(64, a.Cin - (a.dw ? n_tile : chunk) * 64) + 15) >> 4;
+          const int cc = a.dw ? n_tile : chunk;       // channels left in this chunk's source (skip S, or U / the single input)
+          const int krem = CAT && cc < ks ? Cs - cc * 64 : a.Cin - Cs - (cc - ks) * 64;
+          const int ksteps = (min(64, krem) + 15) >> 4;
           const uint32_t a_lo = a_lo0 + (uint32_t)s * a_stage16;
           mbar_wait(&full[s], ph, 2);
           tc_fence_after();
@@ -415,10 +434,14 @@ using namespace b200;
 //        bits 8..15: force grid size = value * 4 CTAs (0 = auto); bits 16..19: pipeline stages wanted (0 = auto);
 //        bits 20..21: CTAs per SM (0 = auto); bit5: never pair M tiles over a shared B stage
 // x: [B,H,W,Cin] input; output [B,Ho,Wo,Cout] with Ho = (H-1)/stride+1.  dwmode: w is the block-diagonal
-// packing bf16 [C][9][64] (see b200seg_dwconv3x3_tc).
-static int launch_conv_tc(const void* x, const void* w, const float* bias, const void* res, void* y, int B, int H,
-                          int W, int Cin, int Cout, int taps, int stride, int dwmode, int act, int flags,
-                          cudaStream_t stream) {
+// packing bf16 [C][9][64] (see b200seg_dwconv3x3_tc).  skip (Cs > 0, stride 1, not dwmode): the input is
+// cat([skip [B,H,W,Cs], x [B,H,W,Cin-Cs]], channel) and w stays [Cout][taps][Cin].  Issued k-steps per tap set
+// equal those of the concatenated input, e.g. the MobileNetV2UNet decoder (Cs + Cu): up1 64 + 1280 -> 84,
+// up2 32 + 256 -> 18, up3 24 + 128 -> 10, up4 16 + 64 -> 5 (conv_rs).
+static int launch_conv_tc(const void* skip, int Cs, const void* x, const void* w, const float* bias, const void* res,
+                          void* y, int B, int H, int W, int Cin, int Cout, int taps, int stride, int dwmode, int act,
+                          int flags, cudaStream_t stream) {
+  const int Cu = Cin - Cs;
   const int Ho = (H - 1) / stride + 1, Wo = (W - 1) / stride + 1;
   ConvTcArgs a;
   a.bias = bias; a.res = res; a.y = y;
@@ -451,8 +474,9 @@ static int launch_conv_tc(const void* x, const void* w, const float* bias, const
       int bn = (((Cout + nt - 1) / nt) + 63) & ~63;
       a.block_n = bn; a.n_tiles = (Cout + bn - 1) / bn;
     }
-    a.k_chunks = (Cin + 63) / 64;
+    a.k_chunks = (Cs + 63) / 64 + (Cu + 63) / 64;
   }
+  a.Cs = Cs; a.ks = (Cs + 63) / 64;
   a.act = act;
   a.tma_store = flags & 1;
   a.halo_bo = (flags & 16) ? 1 : 0;   // measured on B200: the swizzle uses absolute smem address bits, base_offset must stay 0
@@ -502,16 +526,21 @@ static int launch_conv_tc(const void* x, const void* w, const float* bias, const
   B200_REQUIRE(smem <= 227 * 1024, "conv_tc: smem %d too large", smem);
   a.total_tiles = ((a.m_tiles + a.mpair - 1) / a.mpair) * a.n_tiles;
 
-  CUtensorMap tmA, tmB, tmC;
+  CUtensorMap tmA, tmB, tmC, tmS;
   {
-    // the activation map always describes the INPUT tensor; for 1x1 it is the flattened pixel axis
+    // the activation maps always describe the INPUT tensors (U, and S when there is a skip); for 1x1 the pixels
+    // are one flat axis
     const uint64_t iw = taps == 1 ? (uint64_t)a.W : (uint64_t)W, ih = taps == 1 ? 1 : (uint64_t)H, ib = taps == 1 ? 1 : (uint64_t)B;
-    uint64_t dims[4] = {(uint64_t)Cin, iw, ih, ib};
-    uint64_t str[3] = {(uint64_t)Cin * 2, (uint64_t)Cin * 2 * iw, (uint64_t)Cin * 2 * iw * ih};
     uint32_t box[4] = {64, (uint32_t)(a.halo ? 130 : a.BW * stride), (uint32_t)(a.BH * stride), 1};
     uint32_t es[4] = {1, (uint32_t)stride, (uint32_t)stride, 1};
-    int rc = make_tmap_bf16(&tmA, x, 4, dims, str, box, 1, es);
-    if (rc) return rc;
+    for (int src = 0; src < (Cs ? 2 : 1); ++src) {
+      const uint64_t c = (uint64_t)(src ? Cs : Cu);
+      uint64_t dims[4] = {c, iw, ih, ib};
+      uint64_t str[3] = {c * 2, c * 2 * iw, c * 2 * iw * ih};
+      int rc = make_tmap_bf16(src ? &tmS : &tmA, src ? skip : x, 4, dims, str, box, 1, es);
+      if (rc) return rc;
+    }
+    if (!Cs) tmS = tmA;
   }
   {
     uint64_t dims[3] = {(uint64_t)(dwmode ? 64 : Cin), (uint64_t)taps, (uint64_t)Cout};
@@ -531,8 +560,10 @@ static int launch_conv_tc(const void* x, const void* w, const float* bias, const
   cudaGetDevice(&dev);
   static bool attr_set[64] = {false};
   if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return set_error((int)e, "conv_tc: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     attr_set[dev] = true;
   }
@@ -546,8 +577,9 @@ static int launch_conv_tc(const void* x, const void* w, const float* bias, const
   if ((flags >> 8) & 0xff) grid = (long long)((flags >> 8) & 0xff) * 4;
   if (grid > a.total_tiles) grid = a.total_tiles;
   a.pdl_early = pdl_mode() != 3;
-  if (a.mpair == 2) launch_pdl_if(pdl_mode() > 0, conv_tc_kernel<2>, dim3((unsigned)grid), dim3(TC_THREADS), (size_t)smem, stream, tmA, tmB, tmC, a);
-  else launch_pdl_if(pdl_mode() > 0, conv_tc_kernel<1>, dim3((unsigned)grid), dim3(TC_THREADS), (size_t)smem, stream, tmA, tmB, tmC, a);
+  auto* kern = a.mpair == 2 ? (Cs ? conv_tc_kernel<2, true> : conv_tc_kernel<2, false>)
+                            : (Cs ? conv_tc_kernel<1, true> : conv_tc_kernel<1, false>);
+  launch_pdl_if(pdl_mode() > 0, kern, dim3((unsigned)grid), dim3(TC_THREADS), (size_t)smem, stream, tmA, tmB, tmC, tmS, a);
   return check_launch("conv_tc");
 }
 
@@ -559,7 +591,18 @@ extern "C" int b200seg_conv_tc(const void* x, const void* w, const float* bias, 
   B200_REQUIRE(Cout > 0 && Cout % 8 == 0, "conv_tc: Cout=%d must be a positive multiple of 8", Cout);
   B200_REQUIRE(B > 0 && H > 0 && W > 0, "conv_tc: empty tensor");
   B200_REQUIRE(x && w && y, "conv_tc: null pointer");
-  return launch_conv_tc(x, w, bias, res, y, B, H, W, Cin, Cout, taps, 1, 0, act, flags, (cudaStream_t)s);
+  return launch_conv_tc(nullptr, 0, x, w, bias, res, y, B, H, W, Cin, Cout, taps, 1, 0, act, flags, (cudaStream_t)s);
+}
+
+extern "C" int b200seg_conv_tc_cat(const void* skip, const void* x, const void* w, const float* bias, const void* res,
+                                   void* y, int B, int H, int W, int Cs, int Cu, int Cout, int taps, int act, int flags,
+                                   b200seg_stream_t s) {
+  B200_REQUIRE(taps == 1 || taps == 9, "conv_tc_cat: taps=%d (1 or 9)", taps);
+  B200_REQUIRE(Cs >= 0 && Cs % 8 == 0 && Cu > 0 && Cu % 8 == 0, "conv_tc_cat: Cs=%d Cu=%d must be multiples of 8 (Cu > 0)", Cs, Cu);
+  B200_REQUIRE(Cout > 0 && Cout % 8 == 0, "conv_tc_cat: Cout=%d must be a positive multiple of 8", Cout);
+  B200_REQUIRE(B > 0 && H > 0 && W > 0, "conv_tc_cat: empty tensor");
+  B200_REQUIRE(x && w && y && (skip || !Cs), "conv_tc_cat: null pointer");
+  return launch_conv_tc(skip, Cs, x, w, bias, res, y, B, H, W, Cs + Cu, Cout, taps, 1, 0, act, flags, (cudaStream_t)s);
 }
 
 extern "C" int b200seg_dwconv3x3_tc(const void* x, const void* wdiag, const float* bias, void* y, int B, int H,
@@ -568,5 +611,5 @@ extern "C" int b200seg_dwconv3x3_tc(const void* x, const void* wdiag, const floa
   B200_REQUIRE(stride == 1 || stride == 2, "dwconv3x3_tc: stride=%d", stride);
   B200_REQUIRE(B > 0 && H > 0 && W > 0, "dwconv3x3_tc: empty tensor");
   B200_REQUIRE(x && wdiag && y, "dwconv3x3_tc: null pointer");
-  return launch_conv_tc(x, wdiag, bias, nullptr, y, B, H, W, C, C, 9, stride, 1, act, flags, (cudaStream_t)s);
+  return launch_conv_tc(nullptr, 0, x, wdiag, bias, nullptr, y, B, H, W, C, C, 9, stride, 1, act, flags, (cudaStream_t)s);
 }
